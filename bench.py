@@ -1,6 +1,6 @@
 """Headline benchmark: views/sec of one Fast3R ViT-L/512 forward pass over N synthetic 512x368 views.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--views V] [--impl ours|reference|library]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--views V] [--impl ours|reference|library] [--dump-outputs DIR]
 
 * ours, 1 GPU: BASELINE.json configs[1] (N=32 views, 512x368, bf16 tensor-core operands) on one B200 is the
   headline `value`; `config.extra` adds configs[2] (N=320, long-sequence regime) with its own roofline, the
@@ -14,7 +14,9 @@
   the CPU oracle port when oracle/_ref is missing.
 
 One JSON line on stdout (rank 0).  `value` = views/s with inputs resident in HBM; `e2e` = the same metric through
-the reference-facing API `inference()` from pinned host buffers including H2D and D2H.
+the reference-facing API `inference()` from pinned host buffers including H2D and D2H.  `--dump-outputs DIR` writes
+the preds of the last timed headline step (see dump_outputs); the inputs and weights are seeded, so two builds run with
+the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -125,6 +127,27 @@ def make_views(n, device=None, pinned=False, seed0=1234, only=None):
         views.append(dict(img=img, true_shape=np.int32([[H, W]]), idx=i, instance=str(i), dataset="synthetic",
                           label=f"v{i}"))
     return views
+
+
+DUMP_BYTES = 60 * 10 ** 6
+
+
+def dump_outputs(preds, out_dir, seed=0):
+    """Writes the preds of one forward - per key the views stacked, (N, B, H, W[, C]) - as float32 `out_dir/<key>.npy`.
+    When they exceed DUMP_BYTES, every key keeps the same seeded sample of pixel positions, (N, B, P[, C]), so that
+    two builds run with the same arguments can be compared value for value."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    out = {k: torch.stack([p[k] for p in preds]).float() for k, v in preds[0].items()
+           if torch.is_tensor(v) and v.is_floating_point()}
+    total = sum(v.numel() * 4 for v in out.values())
+    for k, v in out.items():
+        if total > DUMP_BYTES:
+            hw = v.shape[2] * v.shape[3]
+            idx = torch.randperm(hw, generator=torch.Generator().manual_seed(seed))[:hw * DUMP_BYTES // total]
+            v = v.flatten(2, 3)[:, :, idx.sort().values.to(v.device)]
+        np.save(os.path.join(out_dir, f"{k}.npy"), v.cpu().numpy())
 
 
 def pick_cpu_threads():
@@ -486,12 +509,13 @@ def run_ours(args, rank, world, local_rank):
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             step()
+        last = step()  # only the last step's preds are kept, so earlier steps allocate exactly as before
         e1.record()
         barrier()
         ops.KERNEL_TIMER = None
-        return e0.elapsed_time(e1) / steps, L.launch_count() - n0, timer
+        return e0.elapsed_time(e1) / steps, L.launch_count() - n0, timer, last
 
     # ================= headline: N = args.views (default 32, BASELINE configs[1]) =================
     N = args.views
@@ -508,8 +532,11 @@ def run_ours(args, rank, world, local_rank):
     sampler.mark()
     if sp is not None:
         sp.timers = []
-    ms, launches, timer = timed_device(views_dev, args.steps, 0)
+    ms, launches, timer, last = timed_device(views_dev, args.steps, 0)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(last, args.dump_outputs)
+    del last
     roof, att_ms = attention_roofline(timer, N, ms, clocks, peak_tf, peak_src)
     sp_trace = None
     if sp is not None and sp.timers:
@@ -589,7 +616,7 @@ def run_ours(args, rank, world, local_rank):
         vd = make_views(n_views, device=dev, only=r)
         if sp is not None:
             sp.timers = []
-        m, _l, tm = timed_device(vd, steps, warmup)
+        m, _l, tm = timed_device(vd, steps, warmup)[:3]
         rf, am = attention_roofline(tm, n_views, m, clocks, peak_tf, peak_src)
         if sp is not None and sp.timers:   # sharded: the attention of a layer = key-range partials + merge (+ exposed wait)
             tr, sp.timers = sp.timers[-DEPTH * steps:], None
@@ -660,10 +687,17 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip config.extra (N=320 / N=1000 / GEMM rates / library bar)")
     ap.add_argument("--no-library-bar", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the preds of the last timed step as DIR/<key>.npy (float32; a seeded pixel sample when "
+                         "the whole output is larger than 60 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return

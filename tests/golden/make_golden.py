@@ -217,7 +217,65 @@ def run_vitl_n4(tag="vitl_n4_368x512", stride=4):
           torch.get_num_threads(), "threads; ref bf16 vs fp32 gap", gap)
 
 
+def run_inference_call(tag="tiny_b1_n3_inference_call"):
+    """The call the reference's own inference(..., dtype="32") makes on the model for the tiny_b1_n3 views: the collated
+    views, the keyword arguments, and the grad / autocast state around it (inference_multiview.py:22-95)."""
+    enc, dec, head = tiny_args()
+    torch.manual_seed(0)
+    model = Fast3R(dict(enc), dict(dec), dict(head)).eval()
+    shapes = {k: tuple(v.shape) for k, v in model.state_dict().items()}
+    model.load_state_dict(synth_state_dict(shapes, seed=0))
+    N, B, H, W = 3, 1, 64, 96
+    imgs = synth_images(N, B, H, W)
+    views = [dict(img=imgs[i], true_shape=np.int32([[H, W]]), idx=i, instance=str(i), dataset="synthetic",
+                  label=f"v{i}") for i in range(N)]
+    calls = []
+
+    def recording_model(vs, **kw):
+        calls.append(dict(views=[{k: v.clone() if torch.is_tensor(v) else v for k, v in x.items()} for x in vs],
+                          kwargs=kw, grad_enabled=torch.is_grad_enabled(),
+                          autocast_enabled=torch.is_autocast_enabled("cpu")))
+        return model(vs, **kw)
+
+    torch.manual_seed(7)
+    inference(views, recording_model, torch.device("cpu"), dtype="32", verbose=False)
+    assert len(calls) == 1
+    torch.save(calls[0], os.path.join(HERE, f"{tag}.pt"))
+    print(tag, "saved", os.path.getsize(os.path.join(HERE, f"{tag}.pt")) / 1e6, "MB", calls[0]["kwargs"])
+
+
+def run_load_images(tag="load_images", n_sample=4096):
+    """The reference's own load_images(dir, size=512) on PNG files (lossless) of seeded random images.  The full fp32
+    outputs are 8 MB, so the fixture keeps per image the true_shape, the sha256 of the full array and a seeded sample
+    of its values."""
+    import hashlib
+    import tempfile
+    from PIL import Image
+    from fast3r.dust3r.utils.image import load_images
+    sizes = [(800, 600), (600, 800), (1024, 1024), (321, 123)]
+    with tempfile.TemporaryDirectory() as d:
+        for i, (w, h) in enumerate(sizes):
+            a = np.random.default_rng(100 + i).integers(0, 256, (h, w, 3), dtype=np.uint8)
+            Image.fromarray(a).save(os.path.join(d, f"im{i}.png"))
+        views = load_images(d, size=512, verbose=False)
+    rng = np.random.default_rng(0)
+    out = []
+    for v in views:
+        img = np.ascontiguousarray(v["img"][0].numpy(), np.float32)
+        idx = np.sort(rng.choice(img.size, n_sample, replace=False))
+        out.append(dict(true_shape=torch.from_numpy(np.asarray(v["true_shape"][0])), shape=tuple(img.shape),
+                        sha256=hashlib.sha256(img.tobytes()).hexdigest(), index=torch.from_numpy(idx),
+                        values=torch.from_numpy(img.reshape(-1)[idx].copy())))
+    torch.save(dict(sizes=sizes, seeds=[100 + i for i in range(len(sizes))], size=512, views=out),
+               os.path.join(HERE, f"{tag}.pt"))
+    print(tag, "saved", os.path.getsize(os.path.join(HERE, f"{tag}.pt")) / 1e6, "MB")
+
+
 if __name__ == "__main__":
+    if len(sys.argv) > 1 and sys.argv[1] == "consumers":
+        run_inference_call()
+        run_load_images()
+        sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "vitl_n4":
         run_vitl_n4()
         sys.exit(0)

@@ -1,6 +1,7 @@
 """Drop-in boundary beyond forward(): hub mixin, config containers, DUSt3R checkpoint loading, portrait views, and the
 reference's own consumers (its inference(), MultiViewDUSt3RLitModule, estimate_camera_poses) running on this model.
-CPU only: the kernels are replaced by tests/abi_emulator.py; tests that need /root/reference skip without it."""
+CPU only: the kernels are replaced by tests/abi_emulator.py.  The Lightning-module test needs the reference fast3r
+package importable and skips without it; the others read fixtures recorded from the reference under tests/golden/."""
 import os
 import sys
 import types
@@ -158,14 +159,20 @@ def _tiny(M, golden_dir, tag="tiny_b1_n3"):
 
 
 def test_reference_inference_function_drives_this_model(emulated, golden_dir):
-    """fast3r.dust3r.inference_multiview.inference (the reference's code, unmodified) with the B200 model object."""
-    _, ref_inference = _reference_or_skip()
+    """The call fast3r.dust3r.inference_multiview.inference (the reference's code, unmodified) makes on the model -
+    collated views, keyword arguments, grad and autocast state, recorded by tests/golden/make_golden.py - replayed on
+    the B200 model object."""
     g, model, views = _tiny(emulated, golden_dir)
+    call = torch.load(os.path.join(golden_dir, "tiny_b1_n3_inference_call.pt"))
+    assert len(call["views"]) == len(views)
+    for v, r in zip(views, call["views"]):
+        assert torch.equal(v["img"], r["img"])
     model.set_precision("fp32")
     torch.manual_seed(g["rng_seed"])
-    res = ref_inference(views, model, torch.device("cpu"), dtype="32", verbose=False)
-    assert sorted(res.keys()) == g["inference_keys"]
-    for p, q in zip(res["preds"], g["preds"]):
+    with torch.set_grad_enabled(call["grad_enabled"]), torch.autocast("cpu", enabled=call["autocast_enabled"]):
+        preds = model(call["views"], **call["kwargs"])
+    assert len(preds) == len(g["preds"])
+    for p, q in zip(preds, g["preds"]):
         for k in q:
             assert rel_l2(p[k], q[k]) < 1e-3, k
 

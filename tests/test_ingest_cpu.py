@@ -1,9 +1,10 @@
 """Image ingest (SURVEY §8 f3), CPU side: the C oracle (oracle/ingest_oracle.c, a restatement of Pillow's 8-bit resampler +
 the crop / normalise of load_images) is pinned bit-exactly against Pillow / torchvision themselves - the third-party
-dependencies the reference calls (fast3r/dust3r/utils/image.py:32, 68-159) - and, when the reference sources are present,
-against the reference's own load_images() on image files; the library's HOST tap-table function is checked against the
-oracle."""
+dependencies the reference calls (fast3r/dust3r/utils/image.py:32, 68-159) - and against what the reference's own
+load_images() returned on image files (a recorded fixture); the library's HOST tap-table function is checked against
+the oracle."""
 import ctypes as C
+import hashlib
 import os
 
 import numpy as np
@@ -60,25 +61,18 @@ def test_full_ingest_matches_pil_torchvision_pipeline(w, h):
         assert np.array_equal(out, ref), (w, h, size, float(np.abs(out - ref).max()))
 
 
-def test_reference_load_images_on_files(tmp_path):
-    """The reference's own load_images() (PNG files, lossless) against the oracle pipeline."""
-    from oracle.ref_harness import reference_available, import_reference
-    if not reference_available():
-        pytest.skip("reference sources not available")
-    import_reference()
-    from fast3r.dust3r.utils.image import load_images
-    from PIL import Image
-    arrs = []
-    for i, (w, h) in enumerate([(800, 600), (600, 800), (1024, 1024), (321, 123)]):
-        a = _img(w, h, 100 + i)
-        Image.fromarray(a).save(tmp_path / f"im{i}.png")
-        arrs.append(a)
-    views = load_images(str(tmp_path), size=512, verbose=False)
-    assert len(views) == len(arrs)
-    for v, a in zip(views, arrs):
-        out, shape = O.ingest(a, 512)
-        assert tuple(v["true_shape"][0]) == tuple(shape)
-        assert np.array_equal(v["img"][0].numpy(), out)
+def test_reference_load_images_on_files(golden_dir):
+    """The reference's own load_images() (PNG files, lossless) against the oracle pipeline.  The fixture, recorded by
+    tests/golden/make_golden.py, holds per image the reference's true_shape, the sha256 of its full fp32 output and a
+    seeded sample of the values."""
+    g = torch.load(os.path.join(golden_dir, "load_images.pt"))
+    assert len(g["views"]) == len(g["sizes"])
+    for (w, h), seed, v in zip(g["sizes"], g["seeds"], g["views"]):
+        out, shape = O.ingest(_img(w, h, seed), g["size"])
+        assert tuple(v["true_shape"].tolist()) == tuple(shape)
+        assert out.shape == v["shape"], (w, h)
+        assert np.array_equal(out.reshape(-1)[v["index"].numpy()], v["values"].numpy()), (w, h)
+        assert hashlib.sha256(np.ascontiguousarray(out, np.float32).tobytes()).hexdigest() == v["sha256"], (w, h)
 
 
 def test_library_tap_tables_match_oracle():

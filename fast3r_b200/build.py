@@ -6,8 +6,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libfast3r_b200.so")
-SOURCES = ["capi.cu", "gemm.cu", "attention.cu", "attention_x3.cu", "elementwise.cu", "ingest.cu", "geometry.cu"]
-HEADERS = ["common.cuh", "f3r_kernels.h", "geometry_math.h", os.path.join("..", "..", "include", "fast3r_b200.h")]
+SOURCES = ["capi.cu", "gemm.cu", "attention.cu", "attention_x3.cu", "elementwise.cu", "ingest.cu", "geometry.cu", "pnp.cu"]
+HEADERS = ["common.cuh", "f3r_kernels.h", "geometry_math.h", "pnp_math.h", os.path.join("..", "..", "include", "fast3r_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC"]
 

@@ -462,6 +462,33 @@ int f3r_focal_weiszfeld(const float* pts, const float* conf, const float* thr, c
                                            static_cast<cudaStream_t>(stream)), "f3r_focal_weiszfeld");
 }
 
+// ---------------------------------------------------------------- camera poses
+static bool pnp_shape_ok(int32_t views, int32_t h, int32_t w, int32_t n_focals, int32_t iters) {
+  return views > 0 && views <= 65535 && h > 0 && w > 0 && static_cast<int64_t>(h) * w <= (1 << 24) && n_focals > 0 &&
+         iters > 0 && static_cast<int64_t>(n_focals) * iters <= (1 << 20);
+}
+
+size_t f3r_pnp_workspace(int32_t views, int32_t h, int32_t w, int32_t n_focals, int32_t iters) {
+  return pnp_shape_ok(views, h, w, n_focals, iters) ? f3r::pnp_workspace(views, h * w, n_focals * iters) : 0;
+}
+
+int f3r_pnp_ransac(const float* pts, const uint8_t* mask, int32_t views, int32_t h, int32_t w, const float* focals,
+                   int32_t n_focals, const float* pp, int32_t iters, int32_t* scores, int32_t* best, double* c2w,
+                   void* workspace, size_t workspace_bytes, void* stream) {
+  if (!pts || !mask || !focals || !scores || !best || !c2w || !workspace) return fail("f3r_pnp_ransac: null operand");
+  if (n_focals < 1) return fail("f3r_pnp_ransac: n_focals must be >= 1");
+  if (iters < 1) return fail("f3r_pnp_ransac: iters must be >= 1");
+  if (!pnp_shape_ok(views, h, w, n_focals, iters))
+    return fail("f3r_pnp_ransac: bad shape (views <= 65535, h*w <= 2^24, n_focals*iters <= 2^20)");
+  if (workspace_bytes < f3r::pnp_workspace(views, h * w, n_focals * iters))
+    return fail("f3r_pnp_ransac: workspace too small (%zu < %zu bytes)", workspace_bytes,
+                f3r::pnp_workspace(views, h * w, n_focals * iters));
+  if (reinterpret_cast<uintptr_t>(workspace) & 255) return fail("f3r_pnp_ransac: workspace not 256-byte aligned");
+  g_launches += 4 + 2 * (f3r::PNP_LM_STEPS + 1);
+  return check(f3r::launch_pnp_ransac(pts, mask, views, h, w, focals, n_focals, pp, iters, scores, best, c2w, workspace,
+                                      static_cast<cudaStream_t>(stream)), "f3r_pnp_ransac");
+}
+
 // ---------------------------------------------------------------- block-level entry points
 size_t f3r_transformer_workspace(int32_t rows, int32_t dim, int32_t hidden) {
   // h [rows, dim] | q [rows, dim] | kv [rows, 2 dim] | att [rows, dim] | hid [rows, hidden], bf16, 256-byte aligned parts

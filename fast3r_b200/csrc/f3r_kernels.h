@@ -106,4 +106,11 @@ size_t focal_workspace(int views);
 cudaError_t launch_focal_weiszfeld(const float* pts, const float* conf, const float* thr, const float* pp, int views,
                                    int H, int W, int iters, float* focal, double* workspace, cudaStream_t stream);
 
+// camera poses (pnp.cu): 4 launches, then PNP_LM_STEPS + 1 refit passes of 2 launches
+constexpr int PNP_LM_STEPS = 10;
+size_t pnp_workspace(int views, int n, int hyps);
+cudaError_t launch_pnp_ransac(const float* pts, const uint8_t* mask, int views, int H, int W, const float* focals,
+                              int n_focals, const float* pp, int iters, int32_t* scores, int32_t* best, double* c2w,
+                              void* workspace, cudaStream_t stream);
+
 }  // namespace f3r

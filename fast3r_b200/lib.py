@@ -47,7 +47,8 @@ EXPORTS = ["f3r_last_error", "f3r_abi_version", "f3r_gemm_desc_size", "f3r_launc
            "f3r_add_f32", "f3r_attention_x3_workspace", "f3r_attention_x3", "f3r_set_option", "f3r_attention_partial",
            "f3r_attention_merge", "f3r_resample_ksize", "f3r_resample_coeffs", "f3r_ingest_rgb8",
            "f3r_transformer_workspace", "f3r_transformer_blocks", "f3r_conf_quantile", "f3r_similarity_fit_workspace",
-           "f3r_similarity_fit", "f3r_similarity_apply", "f3r_focal_workspace", "f3r_focal_weiszfeld"]
+           "f3r_similarity_fit", "f3r_similarity_apply", "f3r_focal_workspace", "f3r_focal_weiszfeld",
+           "f3r_pnp_workspace", "f3r_pnp_ransac"]
 
 _lib = None
 
@@ -97,7 +98,13 @@ def load() -> C.CDLL:
     lib.f3r_focal_workspace.restype = C.c_size_t
     lib.f3r_focal_weiszfeld.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                         C.c_int32, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
-    for name in ("f3r_conf_quantile", "f3r_similarity_fit", "f3r_similarity_apply", "f3r_focal_weiszfeld"):
+    lib.f3r_pnp_workspace.argtypes = [C.c_int32] * 5
+    lib.f3r_pnp_workspace.restype = C.c_size_t
+    lib.f3r_pnp_ransac.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
+                                   C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                   C.c_void_p]
+    for name in ("f3r_conf_quantile", "f3r_similarity_fit", "f3r_similarity_apply", "f3r_focal_weiszfeld",
+                 "f3r_pnp_ransac"):
         getattr(lib, name).restype = C.c_int
     lib.f3r_set_option.argtypes = [C.c_char_p, C.c_int32]
     lib.f3r_set_option.restype = C.c_int

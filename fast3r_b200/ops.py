@@ -361,3 +361,30 @@ def focal_weiszfeld(pts: torch.Tensor, conf: Optional[torch.Tensor] = None, thr:
         L.check(lib.f3r_focal_weiszfeld(_ptr(pts), _ptr(conf), _ptr(thr), _ptr(pp), views, h, w, int(iters), _ptr(focal),
                                         _ptr(ws), nbytes, _stream(pts)), "f3r_focal_weiszfeld")
     return focal
+
+
+# ------------------------------------------------------------------ camera poses (csrc/pnp.cu)
+def pnp_ransac(pts: torch.Tensor, mask: torch.Tensor, focals: torch.Tensor, pp: Optional[torch.Tensor] = None,
+               iters: int = 10):
+    """pts fp32 [views, H, W, 3]; mask uint8 [views, H, W]; focals fp32 [views, n_focals] (candidates per view); pp fp32
+    [views, 2] or None (= (W/2, H/2)).  Per view, `iters` P3P-RANSAC hypotheses per candidate focal, the best refined by
+    Levenberg-Marquardt (f3r_pnp_ransac).  Returns scores int32 [views, n_focals, iters] (inliers at <= 5 px),
+    best int32 [views, 2] = (k, i) of the selected hypothesis or (-1, -1), c2w fp64 [views, 3, 4]."""
+    _chk(pts, F32, "pts"); _chk(mask, torch.uint8, "mask"); _chk(focals, F32, "focals")
+    views, h, w = pts.shape[0], pts.shape[1], pts.shape[2]
+    assert pts.shape == (views, h, w, 3) and mask.shape == (views, h, w)
+    assert focals.dim() == 2 and focals.shape[0] == views
+    n_focals = focals.shape[1]
+    if pp is not None:
+        _chk(pp, F32, "pp")
+        assert pp.shape == (views, 2)
+    lib = L.load()
+    nbytes = int(lib.f3r_pnp_workspace(views, h, w, n_focals, int(iters)))
+    ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=pts.device)  # caching allocator: >= 512-byte aligned
+    scores = torch.empty(views, n_focals, max(int(iters), 0), dtype=torch.int32, device=pts.device)
+    best = torch.empty(views, 2, dtype=torch.int32, device=pts.device)
+    c2w = torch.empty(views, 3, 4, dtype=torch.float64, device=pts.device)
+    with _on_device(pts):
+        L.check(lib.f3r_pnp_ransac(_ptr(pts), _ptr(mask), views, h, w, _ptr(focals), n_focals, _ptr(pp), int(iters),
+                                   _ptr(scores), _ptr(best), _ptr(c2w), _ptr(ws), nbytes, _stream(pts)), "f3r_pnp_ransac")
+    return scores, best, c2w

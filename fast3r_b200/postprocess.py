@@ -11,14 +11,25 @@ Same names, arguments and results as the reference:
   (returns a python float), and ``estimate_focal_knowing_depth(pts3d, pp, focal_mode="weiszfeld")`` -
   fast3r/dust3r/post_process.py:19-79 (returns a (B,) tensor).
 
-NOT here (documented in DESIGN.md §1): fast_pnp / cv2.solvePnPRansac (cloud_opt/init_im_poses.py:300-350) and the
-"median" focal mode.  Tensors may live on the CPU (what ``inference()`` returns) or on a CUDA device; CPU inputs are
+* ``estimate_camera_poses(preds, views=None, niter_PnP=10, focal_length_estimation_method='individual')`` -
+  MultiViewDUSt3RLitModule.estimate_camera_poses (multiview_dust3r_module.py:806-869, :1038-1078) returning
+  ``(poses_c2w_all, estimated_focals_all)``, and ``fast_pnp(pts3d, focal, msk, device=None, pp=None, niter_PnP=10,
+  num_guessed_focals=100)`` - fast3r/dust3r/cloud_opt/init_im_poses.py:300-350.  The reference runs one
+  cv2.solvePnPRansac (SQPnP) per view and candidate focal on the CPU; here every view of a shape goes through one
+  P3P-RANSAC call (csrc/pnp.cu): the same mask (conf > 1), pixel grid, focal candidates, 5 px threshold and
+  first-strictly-best focal, with a Levenberg-Marquardt refit on the inliers in place of SQPnP's.  The inlier test is
+  division-free, so it differs from cv2.projectPoints only for points at depth exactly 0 (never inliers here).  Poses
+  are not bit-identical to OpenCV's (its RANSAC draws from its own generator); they are deterministic.
+
+NOT here (documented in DESIGN.md §1): the "median" focal mode.  Tensors may live on the CPU (what ``inference()`` returns) or on a CUDA device; CPU inputs are
 copied to ``device`` (default cuda:0) and the results copied back, so the function is a drop-in either way.  There is
 no CPU implementation: without the CUDA library this raises.
 """
 from __future__ import annotations
 
 from typing import Dict, List, Optional
+
+import numpy as np
 
 import torch
 
@@ -103,3 +114,107 @@ def estimate_focal_knowing_depth(pts3d: torch.Tensor, pp: torch.Tensor, focal_mo
     dev = _device_of(pts3d, device)
     ppt = _f32(torch.as_tensor(pp), dev).reshape(-1, 2).expand(b, 2).contiguous()
     return ops.focal_weiszfeld(_f32(pts3d, dev), None, None, ppt, iters=10).to(pts3d.device)
+
+
+_FOCAL_METHODS = ("individual", "first_view_from_global_head", "first_view_from_local_head")
+
+
+def _pnp_group(pts: List[torch.Tensor], confs: List[torch.Tensor], focals: List, niter_PnP: int, dev: torch.device):
+    """One f3r_pnp_ransac call over same-shape views.  focals[j]: candidate list (np.float64 array or [float]) of view j.
+    Returns [(pose c2w float32 (4, 4) or None, focal or None)]."""
+    p = torch.stack([_f32(t, dev) for t in pts])
+    m = torch.stack([(c.to(dev) > 1.0) for c in confs]).to(torch.uint8).contiguous()
+    f32 = torch.tensor(np.asarray(focals, dtype=np.float64), dtype=torch.float32).to(dev)
+    _, best, c2w = ops.pnp_ransac(p, m, f32, None, iters=niter_PnP)
+    best, c2w = best.cpu().numpy(), c2w.cpu().numpy()
+    out = []
+    for j in range(len(pts)):
+        k = int(best[j, 0])
+        if k < 0:
+            out.append((None, None))
+            continue
+        pose = np.eye(4, dtype=np.float32)
+        pose[:3] = c2w[j]
+        out.append((pose, focals[j][k]))
+    return out
+
+
+def _candidates(focal, h: int, w: int, num_guessed_focals: int):
+    if focal is None:  # init_im_poses.py:310-312, evaluated in float64
+        s = max(w, h)
+        return np.geomspace(s / 2, s * 3, num=num_guessed_focals)
+    return [focal]
+
+
+def fast_pnp(pts3d: torch.Tensor, focal, msk: torch.Tensor, device=None, pp=None, niter_PnP: int = 10,
+             num_guessed_focals: int = 100):
+    """Pose of one view from its pointmap pts3d (H, W, 3) and boolean mask (H, W): ``(best_focal, c2w)`` with c2w a
+    float32 (4, 4) tensor, or ``(None, None)`` when fewer than 4 pixels are masked or no hypothesis has an inlier.
+    focal None sweeps ``num_guessed_focals`` candidates (np.geomspace(S/2, 3S), S = max(H, W)), otherwise focal is kept.
+    The work runs on pts3d's CUDA device (CPU inputs: on ``device`` if it is a CUDA device, else cuda:0); c2w is
+    returned on ``device`` if given, else on pts3d's device."""
+    if int(msk.sum()) < 4:
+        return None, None
+    h, w, three = pts3d.shape
+    assert three == 3
+    out_dev = torch.device(device) if device is not None else pts3d.device
+    dev = _device_of(pts3d, device if out_dev.type == "cuda" else None)
+    cands = _candidates(focal, h, w, num_guessed_focals)
+    p = _f32(pts3d, dev).unsqueeze(0)
+    m = msk.to(dev).to(torch.uint8).reshape(1, h, w).contiguous()
+    f32 = torch.tensor(np.asarray(cands, dtype=np.float64), dtype=torch.float32).reshape(1, -1).to(dev)
+    ppt = None if pp is None else _f32(torch.as_tensor(pp), dev).reshape(1, 2)
+    _, best, c2w = ops.pnp_ransac(p, m, f32, ppt, iters=niter_PnP)
+    k = int(best[0, 0])
+    if k < 0:
+        return None, None
+    pose = torch.eye(4, dtype=torch.float64)
+    pose[:3] = c2w[0].cpu()
+    return cands[k], pose.to(torch.float32).to(out_dev)
+
+
+def estimate_camera_poses(preds: List[Dict], views=None, niter_PnP: int = 10,
+                          focal_length_estimation_method: str = "individual", device=None):
+    """Camera-to-world pose and focal of every view of every batch item: ``(poses_c2w_all, estimated_focals_all)``,
+    lists over the B batch items of lists over the N views.  A pose is a float32 (4, 4) numpy array; a view whose pose
+    cannot be estimated gets np.eye(4) and focal None.  'individual' sweeps 100 focals per view (niter_PnP hypotheses
+    each); the 'first_view_*' methods estimate one focal per batch item from its first view (estimate_focal,
+    min_conf_thr_percentile=10) and keep it."""
+    batch_size = len(preds[0]["pts3d_in_other_view"])
+    if focal_length_estimation_method not in _FOCAL_METHODS:
+        raise ValueError(f"Unknown focal_length_estimation_method: {focal_length_estimation_method}")
+    key_pts, key_conf = {"first_view_from_global_head": ("pts3d_in_other_view", "conf"),
+                         "first_view_from_local_head": ("pts3d_local_aligned_to_global", "conf_local")}.get(
+        focal_length_estimation_method, (None, None))
+    items = []  # (batch item, view, pts (H, W, 3), conf (H, W), candidate focals)
+    for i in range(batch_size):
+        focal = None
+        if key_pts is not None:
+            focal = estimate_focal(preds[0][key_pts][i].unsqueeze(0), preds[0][key_conf][i].unsqueeze(0),
+                                   min_conf_thr_percentile=10, device=device)
+        for v, pred in enumerate(preds):
+            pts, conf = pred["pts3d_in_other_view"][i], pred["conf"][i]
+            h, w = pts.shape[0], pts.shape[1]
+            items.append((i, v, pts, conf, _candidates(focal, h, w, 100)))
+    results = {}
+    if items:
+        dev = _device_of(items[0][2], device)
+        by_shape: Dict[tuple, list] = {}
+        for it in items:
+            by_shape.setdefault((tuple(it[2].shape), len(it[4])), []).append(it)
+        for group_all in by_shape.values():
+            for g0 in range(0, len(group_all), _GROUP):
+                group = group_all[g0:g0 + _GROUP]
+                res = _pnp_group([it[2] for it in group], [it[3] for it in group], [it[4] for it in group], niter_PnP, dev)
+                for it, r in zip(group, res):
+                    results[(it[0], it[1])] = r
+    poses_c2w_all, estimated_focals_all = [], []
+    for i in range(batch_size):
+        poses, focals = [], []
+        for v in range(len(preds)):
+            pose, f = results[(i, v)]
+            poses.append(np.eye(4) if pose is None else pose)
+            focals.append(f)
+        poses_c2w_all.append(poses)
+        estimated_focals_all.append(focals)
+    return poses_c2w_all, estimated_focals_all

@@ -176,6 +176,24 @@ size_t f3r_focal_workspace(int32_t views);
 int f3r_focal_weiszfeld(const float* pts, const float* conf, const float* thr, const float* pp, int32_t views, int32_t h,
                         int32_t w, int32_t iters, float* focal, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- camera poses (SURVEY §8 f2): fast_pnp (fast3r/dust3r/cloud_opt/init_im_poses.py:300-350), i.e. per view and per
+ * candidate focal a RANSAC PnP over the masked pixels, for all views of one shape in one call.
+ * pts [views][h][w][3] fp32 pointmap, mask [views][h][w] uint8 (non-zero: pixel used), focals [views][n_focals] fp32
+ * candidates, pp [views][2] fp32 principal points or NULL (= (w/2, h/2)).  Pixel (x, y) is the point (x, y): integer
+ * coordinates.  Per view and focal k, `iters` hypotheses i: 4 distinct masked pixels drawn by a fixed counter-based hash
+ * of (k, i, draw), P3P on three, the fourth picks among its solutions.  scores [views][n_focals][iters] int32 = number of
+ * masked pixels with reprojection error <= 5 px under the hypothesis, tested division-free in fp32 as
+ * (P0 X - u P2 X)^2 + (P1 X - v P2 X)^2 <= 25 (P2 X)^2 with P = K [R | t] (a point with P2 X = 0 never counts).
+ * best [views][2] = (k, i) of the highest score, ties to the lowest k then i, or (-1, -1) when every score is 0
+ * (also when fewer than 4 pixels are masked).  The selected pose is refined by Levenberg-Marquardt steps on the
+ * reprojection error over its inliers; c2w [views][3][4] fp64 = its camera-to-world inverse [R^T | -R^T t] (zeros for a
+ * failed view).  workspace: f3r_pnp_workspace(views, h, w, n_focals, iters) bytes, 256-byte aligned.  Deterministic:
+ * results depend neither on scheduling nor on which other views share the call. */
+size_t f3r_pnp_workspace(int32_t views, int32_t h, int32_t w, int32_t n_focals, int32_t iters);
+int f3r_pnp_ransac(const float* pts, const uint8_t* mask, int32_t views, int32_t h, int32_t w, const float* focals,
+                   int32_t n_focals, const float* pp, int32_t iters, int32_t* scores, int32_t* best, double* c2w,
+                   void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- parity mode: the reference's fp32 path (inference_multiview.py:41-49, dtype="32": no autocast) on the bf16
  * tensor pipe.  Every fp32 operand x is carried as hi + lo (two bf16), every product as hi*hi + lo*hi + hi*lo with
  * fp32 accumulation.  For f3r_gemm this is the ordinary kernel over a 3x longer K: A' = f3r_split3(A) = [hi|lo|hi],
